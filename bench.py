@@ -185,7 +185,7 @@ def reference_step_fn(np_dtype, nsamp):
   """One reference step = `nsamp` full <psi|psi> contractions through the reference's OWN code: tn.Node construction,
   edge wiring and `tn.contractors.greedy` (path_contractors.py:36-97,165-193 -> contract_between, network_components.py:1984-2095
   -> NumPyBackend.tensordot, numpy_backend.py:35-54) on backend="numpy", from the unmodified package installed under
-  baseline/_ref (tools/install_ref.sh).  Falls back to the oracle restatement (kind "port") only when that install is absent.
+  oracle/_ref by build().  Falls back to the oracle restatement (kind "port") only when that install is absent.
   Returns (step, kind, one_network)."""
   nets = [[k.astype(np_dtype) for k in make_kets(L_SITES, BOND, PHYS, 3 + b)] for b in range(nsamp)]
   from baseline import refenv  # pylint: disable=import-outside-toplevel
@@ -239,7 +239,7 @@ def reference_measure(np_dtype, nsamp, steps, warmup):
           "result": float(np.real(res)),
           "sample": "%d network(s) per step x %d steps (127 pairwise each) through %s on numpy %s, BLAS threads = %d (fastest of "
                     "8/16/32/64/all on this host; %d logical cores)"
-                    % (nsamp, steps, "the reference's tn.contractors.greedy (baseline/_ref)" if kind == "reference" else
+                    % (nsamp, steps, "the reference's tn.contractors.greedy (oracle/_ref)" if kind == "reference" else
                        "the oracle restatement", np.dtype(np_dtype).name, threads, os.cpu_count())}
 
 
@@ -247,7 +247,7 @@ NP_DTYPE = {"bf16": np.float32, "f32": np.float32, "f64": np.float64}
 
 
 def run_reference(args, rank, world):
-  """The reference arm: the UNMODIFIED reference (baseline/_ref) contracting the same workload on its own numpy backend,
+  """The reference arm: the UNMODIFIED reference (oracle/_ref) contracting the same workload on its own numpy backend,
   all the host threads it can use.  numpy has no bfloat16: for --dtype bf16 the reference computes in float32 (the narrowest
   type its BLAS supports) and the line says so; `by_dtype` carries the float32 AND float64 figures so that every GPU dtype
   has a like-for-like (or wider) reference number."""
@@ -308,7 +308,13 @@ def main():
                   "(no nested sub-records, single BLAS thread setting for the CPU leg)")
   ap.add_argument("--no-strong-scaling", action="store_true", help="N > 1: skip the one-network strong-scaling sub-record")
   ap.add_argument("--no-subrecords", action="store_true", help="skip the by_dtype / configs sub-records of the default line")
+  ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                  help="after the timed steps, write what the last timed step computed (the value of every network, "
+                       "float64) to DIR/result.npy (DIR/result_rank<r>.npy with several ranks); the inputs are seeded, so "
+                       "two builds run with the same arguments can be compared output for output")
   args = ap.parse_args()
+  if args.dump_outputs is not None and (args.config != "cfg2" or args.impl != "cuda_b200"):
+    ap.error("--dump-outputs writes the outputs of the default workload (--config cfg2 --impl cuda_b200)")
   quiet_stdout()
   args.warmup = max(args.warmup, 3) if args.impl == "cuda_b200" else max(args.warmup, 1)
   rank = int(os.environ.get("RANK", "0"))
@@ -411,7 +417,11 @@ def main():
   sampler.window = (win0, time.time())
   launches = (net.launches_per_replay * args.steps) if net is not None else (lib.tnb200_launch_count() - l0)
   ms = e0.elapsed_time(e1)
-  result_value = [float(x) for x in np.atleast_1d(res.to_host().astype(np.float64))]
+  result_host = np.atleast_1d(res.to_host().astype(np.float64))
+  result_value = [float(x) for x in result_host]
+  if args.dump_outputs is not None:
+    os.makedirs(args.dump_outputs, exist_ok=True)
+    np.save(os.path.join(args.dump_outputs, "result.npy" if world == 1 else "result_rank%d.npy" % rank), result_host)
 
   # ---- latency of ONE network (no sample batching): the same plan compiled for a single MPS sample
   single = None
@@ -831,7 +841,7 @@ def kernel_profile(be, dev, labels, path, work, nbatch, nb, esize, reps=3):
 
 
 def cpu_baseline(args):
-  """The reference itself (baseline/_ref, numpy backend; oracle port only if that install is absent) on the host cores,
+  """The reference itself (oracle/_ref, numpy backend; oracle port only if that install is absent) on the host cores,
   bounded sample, at the dtype of this run (float32 for bf16: numpy has no bfloat16)."""
   m = reference_measure(NP_DTYPE[args.dtype], 1, args.cpu_baseline_steps, 1)
   return {"value": m["value"], "unit": "contractions/s", "cores": m["cores"], "kind": m["kind"],
@@ -1167,7 +1177,7 @@ def run_config(args):
         c = rng.standard_normal((dl, 2, dr))
         tensors.append(c / np.linalg.norm(c))
     if tn_ref is None:
-      raise RuntimeError("cfg5 needs the reference driver (baseline/_ref): run tools/install_ref.sh")
+      raise RuntimeError("cfg5 needs the reference driver (oracle/_ref, installed by build())")
 
     def arm(backend, count, sync):
       mps = tn_ref.FiniteMPS([t.copy() for t in tensors], canonicalize=False, backend=backend)

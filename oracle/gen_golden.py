@@ -1,6 +1,6 @@
 """Generate tests/golden/*.npz by running the REAL reference (numpy backend).
 
-Run in the build container only:  python -m oracle.gen_golden
+Needs the reference installed in oracle/_ref (oracle/build_ref.py):  python -m oracle.gen_golden
 Inputs are seeded; every array the reference returned is stored next to its inputs and
 a JSON description of the call, so the fixtures can be replayed against (a) the oracle
 restatement (tests/test_oracle_golden.py, CPU) and (b) the CUDA path (tests -m gpu).
@@ -358,6 +358,41 @@ def gen_dmrg(tn):
   _save("dmrg", meta, arrays)
 
 
+def gen_tree(tn):
+  """tn.contractors.greedy (path_contractors.py:165-193) on backend numpy over a scaled-down copy of bench.py's 32-tensor
+  tree network (the strong-scaling workload), seeded inputs as in tests/test_host_logic_r2.py: the closed network's value."""
+  import bench  # pylint: disable=import-outside-toplevel
+  labels, _, shapes, _ = bench.ttn_network({"b3": 24, "b2": 8, "b1": 4, "p": 3})
+  rng = np.random.default_rng(2)
+  kets = [rng.standard_normal(shapes[i]) / np.sqrt(np.prod(shapes[i][1:])) for i in range(len(labels) // 2)]
+  nodes = [tn.Node(t, backend="numpy") for t in kets + [np.conj(k) for k in kets]]
+  seen = {}
+  for node, labs in zip(nodes, labels):
+    for ax, l in enumerate(labs):
+      if l in seen:
+        seen[l] ^ node[ax]
+      else:
+        seen[l] = node[ax]
+  value = float(tn.contractors.greedy(nodes).tensor)
+  _save("tree", [dict(dims={"b3": 24, "b2": 8, "b1": 4, "p": 3}, seed=2, greedy=value)], {})
+
+
+def gen_ref_callers(tn):
+  """Every case of tests/ref_cases.py (the reference's own callers: Node @, contract_between, ncon, contractors, split_node*,
+  CopyNode / bucket, FiniteMPS, FiniteDMRG) on backend numpy: the arrays tests/test_gpu_reference_callers.py compares the
+  cuda_b200 arm against."""
+  import sys  # pylint: disable=import-outside-toplevel
+  sys.path.insert(0, os.path.dirname(OUT))
+  import ref_cases  # pylint: disable=import-outside-toplevel
+  meta, arrays = [], {}
+  for name, fn, _ in ref_cases.CASES:
+    out = fn(tn, "numpy")
+    for i, a in enumerate(out):
+      arrays["%s__%d" % (name, i)] = np.asarray(a)
+    meta.append(dict(name=name, outputs=len(out)))
+  _save("ref_callers", meta, arrays)
+
+
 def main():
   tn = ref_shim.load()
   assert tn.__version__ == "0.4.6"
@@ -370,6 +405,8 @@ def main():
   gen_blocksparse(tn)
   gen_dmrg(tn)
   gen_symsvd(tn)
+  gen_tree(tn)
+  gen_ref_callers(tn)
 
 
 if __name__ == "__main__":

@@ -2,12 +2,9 @@
 checks that run the reference's own callers.  Test infrastructure.
 
 The import environment (three third-party stand-ins: h5py, graphviz, opt_einsum — SURVEY.md 8c /
-Appendix A.1) lives in baseline/refenv.py; the package itself is the unmodified copy installed by
-tools/install_ref.sh into baseline/_ref (which travels to the GPU box), else /root/reference.
+Appendix A.1) lives in baseline/refenv.py; the package itself is the unmodified copy that oracle/build_ref.py installs into oracle/_ref.
 """
 from baseline import refenv
-
-REF_ROOT = refenv.SOURCE_TREE
 
 
 def available() -> bool:

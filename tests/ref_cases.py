@@ -1,7 +1,7 @@
 """The reference's OWN callers, parametrised by backend name.
 
 Each case builds its inputs from a fixed seed, drives the unmodified reference
-(`baseline/_ref`, loaded through baseline/refenv.py) with `backend=<name>` and returns a list of
+(`oracle/_ref`, loaded through baseline/refenv.py) with `backend=<name>` and returns a list of
 host arrays.  tests/test_gpu_reference_callers.py runs every case with backend="numpy" and
 backend="cuda_b200" (the real libtnb200.so kernels) in the same process and compares;
 tests/refhost_runner.py runs the same cases against the host test double.

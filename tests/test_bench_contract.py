@@ -21,7 +21,7 @@ def test_reference_arm_prints_one_json_line_with_contract_keys():
             "config", "cpu_baseline", "e2e"):
     assert k in d, k
   assert d["vs_baseline"] is None and d["higher_is_better"] is True and d["value"] > 0
-  # baseline/_ref installed (tools/install_ref.sh) -> the unmodified reference times itself; only without it the oracle port
+  # oracle/_ref installed (by build()) -> the unmodified reference times itself; only without it the oracle port
   from baseline import refenv
   assert d["cpu_baseline"]["kind"] == ("reference" if refenv.available() else "port") and d["cpu_baseline"]["cores"] >= 1
   assert set(d["by_dtype"]) == {"f32", "f64"} and all(v["value"] > 0 for v in d["by_dtype"].values())

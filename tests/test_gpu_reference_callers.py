@@ -1,9 +1,10 @@
 """Row N1: the reference's own callers, UNMODIFIED, on backend="cuda_b200" with the real kernels.
 
-The reference package is the pip-installed copy under baseline/_ref (tools/install_ref.sh), imported
+The reference package is the copy build() installs under oracle/_ref (oracle/build_ref.py), imported
 through baseline/refenv.py.  Every case of tests/ref_cases.py is run with backend="numpy" (the
 reference's own numpy backend) and backend="cuda_b200" in the same process, on the same seeded
-inputs, and compared (fp64: <= 1e-10 of the result scale; integers exact)."""
+inputs, and compared (fp64: <= 1e-10 of the result scale; integers exact).  Both arms are also compared with the
+numpy arm's results stored in tests/golden/ref_callers.npz (oracle/gen_golden.py:gen_ref_callers)."""
 import numpy as np
 import pytest
 import ref_cases
@@ -23,13 +24,17 @@ def _backend(tn):
 
 
 @pytest.mark.parametrize("name,fn,tol", ref_cases.CASES, ids=[c[0] for c in ref_cases.CASES])
-def test_reference_caller(tn, name, fn, tol):
+def test_reference_caller(tn, golden, name, fn, tol):
   be = _backend(tn)
   n0 = be.lib.tnb200_launch_count()
   got = fn(tn, "cuda_b200")
   launches = be.lib.tnb200_launch_count() - n0
   ref = fn(tn, "numpy")
   ref_cases.compare(name, got, ref, tol)
+  meta, z = golden("ref_callers")
+  stored = [z["%s__%d" % (name, i)] for i in range(next(m["outputs"] for m in meta if m["name"] == name))]
+  ref_cases.compare(name, ref, stored, tol)
+  ref_cases.compare(name, got, stored, tol)
   assert launches > 0, "no libtnb200 kernel ran for " + name
 
 

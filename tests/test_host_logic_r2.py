@@ -107,31 +107,19 @@ def test_blocksparse_degeneracy_arithmetic():
     np.testing.assert_array_equal(h, ref)
 
 
-def test_strong_scaling_network_oracle_equals_the_reference():
+def test_strong_scaling_network_oracle_equals_the_reference(golden):
   """The strong-scaling record checks the sharded result against the numpy oracle (`oracle.np_network.contract_path`); here the
   oracle itself is pinned, on a scaled-down copy of the same 32-tensor tree network, to the unmodified reference
-  (`tn.contractors.greedy` on backend numpy; build container / any box where baseline/_ref is installed)."""
-  import pytest
-  from baseline import refenv
-  tn = refenv.try_load()
-  if tn is None:
-    pytest.skip("baseline/_ref not installed")
+  (`tn.contractors.greedy` on backend numpy, value stored by oracle/gen_golden.py:gen_tree in tests/golden/tree.npz)."""
   import bench
   from oracle import np_network as nn
-  labels, sizes, shapes, dims = bench.ttn_network({"b3": 24, "b2": 8, "b1": 4, "p": 3})
-  rng = np.random.default_rng(2)
+  meta, _ = golden("tree")
+  dims, seed, ref = meta[0]["dims"], meta[0]["seed"], meta[0]["greedy"]
+  labels, sizes, shapes, _ = bench.ttn_network(dims)
+  rng = np.random.default_rng(seed)
   n_ket = len(labels) // 2
   kets = [rng.standard_normal(shapes[i]) / np.sqrt(np.prod(shapes[i][1:])) for i in range(n_ket)]
   host = kets + [np.conj(k) for k in kets]
   path = nn.greedy_path(labels, [], sizes)
   want = float(nn.contract_path(host, labels, path, []))
-  nodes = [tn.Node(t, backend="numpy") for t in host]
-  seen = {}
-  for node, labs in zip(nodes, labels):
-    for ax, l in enumerate(labs):
-      if l in seen:
-        seen[l] ^ node[ax]
-      else:
-        seen[l] = node[ax]
-  got = float(tn.contractors.greedy(nodes).tensor)
-  assert abs(got - want) <= 1e-12 * abs(want)
+  assert abs(ref - want) <= 1e-12 * abs(want)

@@ -1,4 +1,4 @@
-"""Build-container only (needs /root/reference): the reference's own callers — tn.Node, tn.ncon,
+"""Needs the reference installed in oracle/_ref by build(): the reference's own callers — tn.Node, tn.ncon,
 contractors.greedy, split_node*, FiniteDMRG.run_two_site — run UNCHANGED on backend="cuda_b200".
 The device layer is replaced by tests/fake_lib.py (host memory + numpy oracle), so this exercises
 the adapter's host logic and the registration path; the kernels are checked by the -m gpu tests."""
@@ -10,7 +10,7 @@ from oracle import ref_shim
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 pytestmark = [pytest.mark.refhost,
-              pytest.mark.skipif(not ref_shim.available(), reason="/root/reference not present (GPU box)")]
+              pytest.mark.skipif(not ref_shim.available(), reason="reference not installed in oracle/_ref")]
 
 
 def _run(*extra):
