@@ -47,7 +47,9 @@ typedef enum {
   TNB200_C64 = 4,   /* interleaved (re, im) float  */
   TNB200_C128 = 5,  /* interleaved (re, im) double */
   TNB200_I32 = 6,
-  TNB200_I64 = 7
+  TNB200_I64 = 7,
+  TNB200_BOOL = 8   /* 1 byte, 0 or 1: masks.  Accepted by copy, compare and masked_fill only; every other entry point
+                       returns TNB200_ERR_DTYPE for it */
 } tnb200_dtype_t;
 
 /* A strided view of device memory.  Strides are in ELEMENTS (like torch), may be 0
@@ -143,6 +145,18 @@ TNB200_API int32_t tnb200_trace(const tnb200_tensor_t* a, const tnb200_tensor_t*
 TNB200_API int32_t tnb200_diagflat(const tnb200_tensor_t* a, const tnb200_tensor_t* c, int64_t k,
                         void* stream);
 
+/* ---- masks: NumPyBackend.index_update (numpy_backend.py:548-552) and the elementwise `<=` InfiniteMPS.canonicalize
+ * builds its mask with (matrixproductstates/infinite_mps.py:239,273).
+ * compare: c = a (op) b for real dtypes, c TNB200_BOOL; a, b, c same shape (0-strides broadcast), a and b one dtype.
+ * masked_fill: out = mask ? value : src (one launch); src / out one dtype (bool included), mask TNB200_BOOL, all one shape
+ * (0-strides broadcast).  The value is (re, im) from the host, or read on the device from value_dev (dtype value_dtype)
+ * when value_dev is not NULL: no host sync either way. */
+typedef enum { TNB200_LT = 0, TNB200_LE = 1, TNB200_GT = 2, TNB200_GE = 3 } tnb200_cmpop_t;
+TNB200_API int32_t tnb200_compare(int32_t op, const tnb200_tensor_t* a, const tnb200_tensor_t* b, const tnb200_tensor_t* c,
+                                  void* stream);
+TNB200_API int32_t tnb200_masked_fill(const tnb200_tensor_t* src, const tnb200_tensor_t* mask, const tnb200_tensor_t* out,
+                                      double re, double im, const void* value_dev, int32_t value_dtype, void* stream);
+
 /* ---- a4: decompositions.svd (backends/numpy/decompositions.py:21-74).
  * Thin SVD of the m x n matrix view `a` (any strides) by one-sided Jacobi:
  *   u (m x r), s (r, real dtype, DESCENDING), vh (r x n), r = min(m, n); all preallocated and
@@ -163,6 +177,25 @@ TNB200_API int32_t tnb200_svd_truncation_count(const tnb200_tensor_t* s, int64_t
  * composed by the adapter. */
 TNB200_API int32_t tnb200_qr(const tnb200_tensor_t* a, const tnb200_tensor_t* q, const tnb200_tensor_t* r,
                   int32_t non_negative_diagonal, void* stream);
+
+/* ---- NumPyBackend.eigh (numpy_backend.py:165-166 = np.linalg.eigh, UPLO='L').  a: (..., n, n), any strides, f32 / f64 /
+ * c64 / c128; only its lower triangle is read and the imaginary part of its diagonal is ignored.  w (..., n): eigenvalues
+ * ascending, in the real dtype; v (..., n, n): eigenvectors as columns, in the input dtype.  Cyclic two-sided Jacobi:
+ * n <= 64 -> one CTA per matrix, the whole stack in one launch; larger n -> blocked Jacobi on the block-pair tournament of
+ * tnb200_svd, convergence decided on the device.  No host synchronisation (graph-capturable).  `info_dev` (device int32[4],
+ * may be NULL): [0] the most sweeps any matrix used, [1] 1 if every matrix converged. */
+TNB200_API int32_t tnb200_eigh(const tnb200_tensor_t* a, const tnb200_tensor_t* w, const tnb200_tensor_t* v, int32_t* info_dev,
+                               void* stream);
+/* ---- NumPyBackend.inv (numpy_backend.py:554-558 = np.linalg.inv).  out = a^-1 for a square n x n view (any strides,
+ * f32 / f64 / c64 / c128) by Gauss-Jordan elimination with partial pivoting.  *info_dev (device int32, required) is set to
+ * 0, or to k + 1 when the pivot of step k is exactly zero (singular matrix; out is then undefined). */
+TNB200_API int32_t tnb200_inv(const tnb200_tensor_t* a, const tnb200_tensor_t* out, int32_t* info_dev, void* stream);
+/* ---- the orthogonalisation of one Arnoldi step (NumPyBackend.eigs, numpy_backend.py:216-291; tensornetwork_b200/arnoldi.py).
+ * basis: (rows, n) row-major contiguous; w: (n,), any stride, basis dtype (f32 / f64 / c64 / c128); 0 <= k < rows.
+ * Classical Gram-Schmidt with one reorthogonalisation of w against basis rows 0..k-1, deterministic reductions; writes
+ * w_perp / |w_perp| into basis row k (zeros if |w_perp| = 0) and h_dev[0..k) = <row j, w> (both passes), h_dev[k] = |w_perp|
+ * (device, basis dtype).  Four launches, no host sync. */
+TNB200_API int32_t tnb200_krylov_orth(const tnb200_tensor_t* basis, const tnb200_tensor_t* w, int32_t k, void* h_dev, void* stream);
 
 /* ---- a11: block_sparse.tensordot per-sector loop (block_sparse/blocksparsetensor.py:1094-1101).
  * For each sector q: C.data[c_map[q]] = A.data[a_map[q]].reshape(m_q,k_q) @ B.data[b_map[q]]

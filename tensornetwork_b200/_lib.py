@@ -12,12 +12,13 @@ MAX_NDIM = 16
 LIB_PATH = os.path.join(os.path.dirname(os.path.abspath(__file__)), "lib", "libtnb200.so")
 
 # dtype codes of tnb200_dtype_t
-F64, F32, F16, BF16, C64, C128, I32, I64 = range(8)
+F64, F32, F16, BF16, C64, C128, I32, I64, BOOL = range(9)
 # status codes
 OK, ERR_INVALID, ERR_DTYPE, ERR_CUDA, ERR_UNSUPPORTED, ERR_NOCONV = 0, -1, -2, -3, -4, -5
 # ops
 ADD, SUB, MUL, DIV, POW = range(5)
 CONJ, SQRT, ABS, NEG, EXP, LOG, SIN, COS, SIGN, REAL, IMAG = range(11)
+LT, LE, GT, GE = range(4)
 CONJ_A, CONJ_B = 1, 2
 MATH_DEFAULT, MATH_STRICT, MATH_SIMT = 0 << 4, 1 << 4, 2 << 4
 
@@ -74,6 +75,11 @@ SIGNATURES = {
     "tnb200_chain_create": (_i32, [_i32, ctypes.POINTER(ChainStep), _pi32, ctypes.POINTER(_vp)]),
     "tnb200_chain_launch": (_i32, [_vp, _vp]),
     "tnb200_chain_destroy": (_i32, [_vp]),
+    "tnb200_compare": (_i32, [_i32, _P, _P, _P, _vp]),
+    "tnb200_masked_fill": (_i32, [_P, _P, _P, _dbl, _dbl, _vp, _i32, _vp]),
+    "tnb200_eigh": (_i32, [_P, _P, _P, _vp, _vp]),
+    "tnb200_inv": (_i32, [_P, _P, _vp, _vp]),
+    "tnb200_krylov_orth": (_i32, [_P, _P, _i32, _vp, _vp]),
 }
 
 _lib = None

@@ -654,6 +654,103 @@ class CudaB200Backend(_Base):
     return lanczos.eigsh_lanczos(self, A, args, initial_state, shape, dtype, num_krylov_vecs,
                                  numeig, tol, delta, ndiag, reorthogonalize)
 
+  # ------------------------------------------------------------------ InfiniteMPS: eigh / eigs / inv / masks
+  def eigh(self, matrix):
+    """numpy_backend.py:165-166 (np.linalg.eigh, UPLO='L'): (w ascending, real dtype; v, eigenvectors as columns)."""
+    return self._eigh(matrix)
+
+  def _eigh(self, matrix, info=None):
+    """eigh with an optional device int32[4] `info` ([0] sweeps, [1] converged flag); None: no host synchronisation."""
+    self._check_type(matrix)
+    if matrix.ndim < 2:
+      raise np.linalg.LinAlgError("{}-dimensional array given. Array must be at least "
+                                  "two-dimensional".format(matrix.ndim))
+    if matrix.shape[-1] != matrix.shape[-2]:
+      raise np.linalg.LinAlgError("Last 2 dimensions of the array must be square")
+    if matrix.code not in (L.F32, L.F64, L.C64, L.C128):
+      raise TypeError("eigh needs a float32/float64/complex tensor")
+    w = self._new(matrix.shape[:-1], T.real_code(matrix.code))
+    v = self._new(matrix.shape, matrix.code)
+    L.check(self.lib.tnb200_eigh(matrix.ref(), w.ref(), v.ref(), None if info is None else info.data_ptr(),
+                                 self._stream()))
+    return w, v
+
+  def inv(self, matrix):
+    """numpy_backend.py:554-558 (np.linalg.inv).  The one D2H of the singularity word makes it uncapturable."""
+    self._check_type(matrix)
+    if len(matrix.shape) > 2:
+      raise ValueError("input to numpy backend method `inv` has shape {}."
+                       " Only matrices are supported.".format(matrix.shape))
+    if matrix.ndim < 2:
+      raise np.linalg.LinAlgError("{}-dimensional array given. Array must be at least "
+                                  "two-dimensional".format(matrix.ndim))
+    if matrix.shape[0] != matrix.shape[1]:
+      raise np.linalg.LinAlgError("Last 2 dimensions of the array must be square")
+    if matrix.code in (L.I32, L.I64):          # np.linalg.inv computes integer input in float64
+      matrix = self.astype(matrix, L.F64)
+    if matrix.code not in (L.F32, L.F64, L.C64, L.C128):
+      raise TypeError("inv needs a float32/float64/complex tensor")
+    self._no_capture("inv")
+    out = self._new(matrix.shape, matrix.code)
+    info = self.torch.empty((), dtype=self.torch.int32, device=self.device)
+    L.check(self.lib.tnb200_inv(matrix.ref(), out.ref(), info.data_ptr(), self._stream()))
+    if int(info.item()) != 0:
+      raise np.linalg.LinAlgError("Singular matrix")
+    return out
+
+  def compare(self, op, x, y):
+    """x (op) y with numpy broadcasting -> device bool tensor (op: _lib.LT / LE / GT / GE)."""
+    if not isinstance(x, B200Tensor):
+      x = self._as_tensor(x, y.code)
+    y = self._as_tensor(y, x.code)
+    code = self._promote(x.code, y.code)
+    if T.is_complex_code(code):
+      raise TypeError("'<' / '<=' / '>' / '>=' are not supported for complex tensors")
+    x, y = self.astype(x, code), self.astype(y, code)
+    try:
+      shape = tuple(np.broadcast_shapes(x.shape, y.shape))
+    except ValueError as e:
+      raise ValueError("operands could not be broadcast together with shapes {} {}".format(
+          x.shape, y.shape)) from e
+    xe = x if x.shape == shape else B200Tensor(x.t.expand(shape), code)
+    ye = y if y.shape == shape else B200Tensor(y.t.expand(shape), code)
+    out = self._new(shape, L.BOOL)
+    L.check(self.lib.tnb200_compare(op, xe.ref(), ye.ref(), out.ref(), self._stream()))
+    return out
+
+  def index_update(self, tensor, mask, assignee):
+    """numpy_backend.py:548-552: a copy of `tensor` with `assignee` (a scalar, or a size-1 device tensor read on the
+    device) at the positions where the boolean `mask` is set.  A host numpy mask is uploaded."""
+    self._check_type(tensor)
+    if isinstance(mask, np.ndarray):
+      mask = self.convert_to_tensor(np.asarray(mask, dtype=np.bool_))
+    self._check_type(mask, "mask")
+    if mask.code != L.BOOL:
+      raise TypeError("index_update needs a boolean mask, got dtype {}".format(mask.dtype))
+    if mask.shape != tensor.shape:
+      try:
+        mask = B200Tensor(mask.t.expand(tensor.shape), L.BOOL)
+      except RuntimeError as e:
+        raise IndexError("boolean index of shape {} does not match the indexed tensor of shape {}".format(
+            mask.shape, tensor.shape)) from e
+    out = self._new(tensor.shape, tensor.code)
+    if isinstance(assignee, B200Tensor):
+      if assignee.size != 1:
+        raise ValueError("index_update: the assignee must be a scalar, got shape {}".format(assignee.shape))
+      L.check(self.lib.tnb200_masked_fill(tensor.ref(), mask.ref(), out.ref(), 0.0, 0.0, assignee.t.data_ptr(),
+                                          assignee.code, self._stream()))
+    else:
+      v = complex(np.asarray(assignee).item())
+      L.check(self.lib.tnb200_masked_fill(tensor.ref(), mask.ref(), out.ref(), v.real, v.imag, None, 0,
+                                          self._stream()))
+    return out
+
+  def eigs(self, A, args=None, initial_state=None, shape=None, dtype=None, num_krylov_vecs=50, numeig=6,
+           tol=1e-8, which='LR', maxiter=None):
+    """numpy_backend.py:216-291 (scipy.sparse.linalg.eigs / ARPACK there): thick-restart Arnoldi, arnoldi.py."""
+    from . import arnoldi  # pylint: disable=import-outside-toplevel
+    return arnoldi.eigs(self, A, args, initial_state, shape, dtype, num_krylov_vecs, numeig, tol, which, maxiter)
+
 
 def register():
   """Insert the backend into the reference's registry (backend_factory.py:22-28)."""

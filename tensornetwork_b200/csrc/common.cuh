@@ -58,13 +58,14 @@ inline int dtype_size(int dt) {
     case TNB200_C128: return 16;
     case TNB200_I32: return 4;
     case TNB200_I64: return 8;
+    case TNB200_BOOL: return 1;
   }
   return 0;
 }
 inline bool dtype_is_complex(int dt) { return dt == TNB200_C64 || dt == TNB200_C128; }
 inline const char* dtype_name(int dt) {
-  static const char* n[] = {"f64", "f32", "f16", "bf16", "c64", "c128", "i32", "i64"};
-  return (dt >= 0 && dt < 8) ? n[dt] : "?";
+  static const char* n[] = {"f64", "f32", "f16", "bf16", "c64", "c128", "i32", "i64", "bool"};
+  return (dt >= 0 && dt < 9) ? n[dt] : "?";
 }
 
 inline int num_sms() {
@@ -230,7 +231,7 @@ __device__ __forceinline__ int64_t mode_offset0(const DevModes& m, int64_t lin) 
 
 inline bool valid_tensor(const tnb200_tensor_t* t) {
   if (!t || t->ndim < 0 || t->ndim > TNB200_MAX_NDIM) return false;
-  if (t->dtype < 0 || t->dtype > TNB200_I64) return false;
+  if (t->dtype < 0 || t->dtype > TNB200_BOOL) return false;
   for (int i = 0; i < t->ndim; ++i) if (t->shape[i] < 0) return false;
   return true;
 }

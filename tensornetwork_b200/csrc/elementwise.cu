@@ -19,6 +19,7 @@ template <> __device__ inline ZV ld<cuFloatComplex>(const cuFloatComplex* p) { c
 template <> __device__ inline ZV ld<cuDoubleComplex>(const cuDoubleComplex* p) { cuDoubleComplex v = *p; return {v.x, v.y}; }
 template <> __device__ inline ZV ld<int32_t>(const int32_t* p) { return {(double)*p, 0.0}; }
 template <> __device__ inline ZV ld<long long>(const long long* p) { return {(double)*p, 0.0}; }
+template <> __device__ inline ZV ld<bool>(const bool* p) { return {*p ? 1.0 : 0.0, 0.0}; }
 
 template <typename T> __device__ inline void stv(T* p, ZV v);
 template <> __device__ inline void stv<double>(double* p, ZV v) { *p = v.re; }
@@ -29,6 +30,7 @@ template <> __device__ inline void stv<cuFloatComplex>(cuFloatComplex* p, ZV v) 
 template <> __device__ inline void stv<cuDoubleComplex>(cuDoubleComplex* p, ZV v) { *p = make_cuDoubleComplex(v.re, v.im); }
 template <> __device__ inline void stv<int32_t>(int32_t* p, ZV v) { *p = (int32_t)llrint(v.re); }
 template <> __device__ inline void stv<long long>(long long* p, ZV v) { *p = llrint(v.re); }
+template <> __device__ inline void stv<bool>(bool* p, ZV v) { *p = v.re != 0.0 || v.im != 0.0; }
 
 #define TNB_DISPATCH_DTYPE(dt, FN, ...)                                           \
   switch (dt) {                                                                   \
@@ -161,6 +163,7 @@ static int copy_from(const tnb200_tensor_t* src, const tnb200_tensor_t* dst, int
     case TNB200_C128: TNB_CP(cuDoubleComplex); break;
     case TNB200_I32: TNB_CP(int32_t); break;
     case TNB200_I64: TNB_CP(long long); break;
+    case TNB200_BOOL: TNB_CP(bool); break;
     default: set_error("copy: bad dtype"); return TNB200_ERR_DTYPE;
   }
 #undef TNB_CP
@@ -175,6 +178,7 @@ int copy_strided(const tnb200_tensor_t* src, const tnb200_tensor_t* dst, int con
     if (src->shape[i] != dst->shape[i]) { set_error("copy: shape mismatch on axis %d", i); return TNB200_ERR_INVALID; }
   if (numel(src) == 0) return 0;
   bool cj = conj && dtype_is_complex(src->dtype);
+  if (src->dtype == TNB200_BOOL) return dst->dtype == TNB200_BOOL ? copy_same<bool>(src, dst, st) : copy_from<bool>(src, dst, 0, st);
   if (src->dtype == dst->dtype && !cj) { TNB_DISPATCH_DTYPE(src->dtype, copy_same, src, dst, st); }
   TNB_DISPATCH_DTYPE(src->dtype, copy_from, src, dst, cj ? 1 : 0, st);
 }
@@ -627,6 +631,66 @@ static int gather_t(const void* src, const int64_t* idx, void* dst, int64_t n, i
   return 0;
 }
 
+// ---------------------------------------------------------------------- masks (TNB200_BOOL)
+// c = a (op) b elementwise for real dtypes, c bool; 0-strides express broadcasting
+template <typename T>
+__global__ void compare_kernel(int op, const T* __restrict__ a, const T* __restrict__ b, bool* __restrict__ c, DevModes m, int64_t total) {
+  for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x) {
+    int64_t o0, o1, o2;
+    mode_offsets3(m, i, o0, o1, o2);
+    const auto x = to_acc(a[o0]), y = to_acc(b[o1]);
+    c[o2] = op == TNB200_LT ? x < y : op == TNB200_LE ? x <= y : op == TNB200_GT ? x > y : x >= y;
+  }
+}
+template <typename T>
+static int compare_t(int op, const tnb200_tensor_t* a, const tnb200_tensor_t* b, const tnb200_tensor_t* c, cudaStream_t st) {
+  DevModes dm; int64_t total;
+  int rc = build_modes(a, b, c, dm, total);
+  if (rc) return rc;
+  if (total == 0) return 0;
+  compare_kernel<T><<<grid_for(total), 256, 0, st>>>(op, (const T*)a->data, (const T*)b->data, (bool*)c->data, dm, total);
+  TNB_LAUNCH_CHECK();
+  count_launch();
+  return 0;
+}
+__device__ inline ZV ld_any(const void* p, int dt) {
+  switch (dt) {
+    case TNB200_F64: return ld<double>((const double*)p);
+    case TNB200_F32: return ld<float>((const float*)p);
+    case TNB200_F16: return ld<__half>((const __half*)p);
+    case TNB200_BF16: return ld<__nv_bfloat16>((const __nv_bfloat16*)p);
+    case TNB200_C64: return ld<cuFloatComplex>((const cuFloatComplex*)p);
+    case TNB200_C128: return ld<cuDoubleComplex>((const cuDoubleComplex*)p);
+    case TNB200_I32: return ld<int32_t>((const int32_t*)p);
+    case TNB200_I64: return ld<long long>((const long long*)p);
+    default: return ld<bool>((const bool*)p);
+  }
+}
+// out = mask ? value : src; the value is given on the host or read on the device (value_dev, value_dt)
+template <typename T>
+__global__ void masked_fill_kernel(const T* __restrict__ src, const bool* __restrict__ mask, T* __restrict__ out, DevModes m, int64_t total,
+                                   ZV value, const void* value_dev, int value_dt) {
+  if (value_dev) value = ld_any(value_dev, value_dt);
+  for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x) {
+    int64_t o0, o1, o2;
+    mode_offsets3(m, i, o0, o1, o2);
+    if (mask[o1]) stv<T>(out + o2, value); else out[o2] = src[o0];
+  }
+}
+template <typename T>
+static int masked_fill_t(const tnb200_tensor_t* src, const tnb200_tensor_t* mask, const tnb200_tensor_t* out, ZV value, const void* value_dev,
+                         int value_dt, cudaStream_t st) {
+  DevModes dm; int64_t total;
+  int rc = build_modes(src, mask, out, dm, total);
+  if (rc) return rc;
+  if (total == 0) return 0;
+  masked_fill_kernel<T><<<grid_for(total), 256, 0, st>>>((const T*)src->data, (const bool*)mask->data, (T*)out->data, dm, total, value,
+                                                         value_dev, value_dt);
+  TNB_LAUNCH_CHECK();
+  count_launch();
+  return 0;
+}
+
 static int real_dtype(int dt) {
   if (dt == TNB200_C128) return TNB200_F64;
   if (dt == TNB200_C64) return TNB200_F32;
@@ -659,6 +723,7 @@ int32_t tnb200_unary(int32_t op, const tnb200_tensor_t* a, const tnb200_tensor_t
   TNB_REQUIRE(valid_tensor(a) && valid_tensor(c), TNB200_ERR_INVALID, "unary: invalid tensor descriptor");
   TNB_REQUIRE(a->ndim == c->ndim, TNB200_ERR_INVALID, "unary: rank mismatch");
   TNB_REQUIRE(op >= TNB200_CONJ && op <= TNB200_IMAG, TNB200_ERR_INVALID, "unary: bad op %d", op);
+  TNB_REQUIRE(a->dtype != TNB200_BOOL && c->dtype != TNB200_BOOL, TNB200_ERR_DTYPE, "unary: bool tensors are not supported");
   cudaStream_t st = (cudaStream_t)stream;
   bool to_real = (op == TNB200_ABS || op == TNB200_REAL || op == TNB200_IMAG) && dtype_is_complex(a->dtype);
   if (to_real) {
@@ -784,6 +849,37 @@ int32_t tnb200_trace(const tnb200_tensor_t* a, const tnb200_tensor_t* c, int64_t
   int64_t base = r0 * a->stride[axis1] + c0 * a->stride[axis2];
   merge_modes(keep, 2);
   TNB_DISPATCH_DTYPE(a->dtype, sum_axes_t, a->data, c->data, keep, rm, base, (cudaStream_t)stream);
+}
+
+int32_t tnb200_compare(int32_t op, const tnb200_tensor_t* a, const tnb200_tensor_t* b, const tnb200_tensor_t* c, void* stream) {
+  TNB_REQUIRE(valid_tensor(a) && valid_tensor(b) && valid_tensor(c), TNB200_ERR_INVALID, "compare: invalid tensor descriptor");
+  TNB_REQUIRE(a->ndim == b->ndim && a->ndim == c->ndim, TNB200_ERR_INVALID, "compare: rank mismatch");
+  TNB_REQUIRE(op >= TNB200_LT && op <= TNB200_GE, TNB200_ERR_INVALID, "compare: bad op %d", op);
+  TNB_REQUIRE(a->dtype == b->dtype, TNB200_ERR_DTYPE, "compare: dtype mismatch");
+  TNB_REQUIRE(c->dtype == TNB200_BOOL, TNB200_ERR_DTYPE, "compare: the output must be bool");
+  cudaStream_t st = (cudaStream_t)stream;
+  switch (a->dtype) {
+    case TNB200_F64: return compare_t<double>(op, a, b, c, st);
+    case TNB200_F32: return compare_t<float>(op, a, b, c, st);
+    case TNB200_F16: return compare_t<__half>(op, a, b, c, st);
+    case TNB200_BF16: return compare_t<__nv_bfloat16>(op, a, b, c, st);
+    case TNB200_I32: return compare_t<int32_t>(op, a, b, c, st);
+    case TNB200_I64: return compare_t<long long>(op, a, b, c, st);
+    default: set_error("compare: dtype %s has no order", dtype_name(a->dtype)); return TNB200_ERR_DTYPE;
+  }
+}
+
+int32_t tnb200_masked_fill(const tnb200_tensor_t* src, const tnb200_tensor_t* mask, const tnb200_tensor_t* out, double re, double im,
+                           const void* value_dev, int32_t value_dtype, void* stream) {
+  TNB_REQUIRE(valid_tensor(src) && valid_tensor(mask) && valid_tensor(out), TNB200_ERR_INVALID, "masked_fill: invalid tensor descriptor");
+  TNB_REQUIRE(src->ndim == mask->ndim && src->ndim == out->ndim, TNB200_ERR_INVALID, "masked_fill: rank mismatch");
+  TNB_REQUIRE(mask->dtype == TNB200_BOOL, TNB200_ERR_DTYPE, "masked_fill: the mask must be bool");
+  TNB_REQUIRE(src->dtype == out->dtype, TNB200_ERR_DTYPE, "masked_fill: dtype mismatch");
+  TNB_REQUIRE(!value_dev || (value_dtype >= TNB200_F64 && value_dtype <= TNB200_BOOL), TNB200_ERR_DTYPE, "masked_fill: bad value dtype");
+  cudaStream_t st = (cudaStream_t)stream;
+  const ZV v{re, im};
+  if (src->dtype == TNB200_BOOL) return masked_fill_t<bool>(src, mask, out, v, value_dev, value_dtype, st);
+  TNB_DISPATCH_DTYPE(src->dtype, masked_fill_t, src, mask, out, v, value_dev, value_dtype, st);
 }
 
 }  // extern "C"

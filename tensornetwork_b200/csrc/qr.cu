@@ -498,6 +498,7 @@ extern "C" int32_t tnb200_qr(const tnb200_tensor_t* a, const tnb200_tensor_t* q,
   const int64_t m = a->shape[0], n = a->shape[1], k = m < n ? m : n;
   TNB_REQUIRE(q->shape[0] == m && q->shape[1] == k && r->shape[0] == k && r->shape[1] == n, TNB200_ERR_INVALID,
               "qr: output shapes must be (m,k), (k,n) with k = min(m,n)");
+  TNB_REQUIRE(a->dtype != TNB200_BOOL, TNB200_ERR_DTYPE, "qr: bool tensors are not supported");
   TNB_REQUIRE(q->dtype == a->dtype && r->dtype == a->dtype, TNB200_ERR_DTYPE, "qr: dtype mismatch");
   TNB_REQUIRE(m < (1LL << 31) && n < (1LL << 31), TNB200_ERR_UNSUPPORTED, "qr: matrix too large");
   set_kernel_name("qr_householder");

@@ -296,6 +296,7 @@ int build_modes(const tnb200_tensor_t* a, const tnb200_tensor_t* b, const tnb200
                 const int32_t* batch_b, ModeList& mB, ModeList& mM, ModeList& mN, ModeList& mK) {
   TNB_REQUIRE(valid_tensor(a) && valid_tensor(b) && valid_tensor(c), TNB200_ERR_INVALID,
               "tensordot: invalid tensor descriptor");
+  TNB_REQUIRE(a->dtype != TNB200_BOOL, TNB200_ERR_DTYPE, "tensordot: bool tensors are not supported");
   TNB_REQUIRE(a->dtype == b->dtype && a->dtype == c->dtype, TNB200_ERR_DTYPE,
               "tensordot: dtype mismatch (%s, %s -> %s)", dtype_name(a->dtype), dtype_name(b->dtype),
               dtype_name(c->dtype));

@@ -9,6 +9,7 @@ callers pass dtypes back to `backend.zeros/randn` as numpy dtypes — SURVEY 8b)
 (device -> host copy) so `np.testing.assert_allclose(node.tensor, ...)` works unchanged.
 """
 import ctypes
+import operator
 import numpy as np
 from . import _lib as L
 
@@ -33,7 +34,7 @@ bfloat16 = BFloat16()
 
 _NP2CODE = {np.dtype(np.float64): L.F64, np.dtype(np.float32): L.F32, np.dtype(np.float16): L.F16,
             np.dtype(np.complex64): L.C64, np.dtype(np.complex128): L.C128,
-            np.dtype(np.int32): L.I32, np.dtype(np.int64): L.I64}
+            np.dtype(np.int32): L.I32, np.dtype(np.int64): L.I64, np.dtype(np.bool_): L.BOOL}
 _CODE2NP = {v: k for k, v in _NP2CODE.items()}
 _CODE2NP[L.BF16] = bfloat16
 _REAL_OF = {L.C64: L.F32, L.C128: L.F64}
@@ -49,7 +50,7 @@ def _init_torch():
     _torch = torch
     _CODE2TORCH = {L.F64: torch.float64, L.F32: torch.float32, L.F16: torch.float16,
                    L.BF16: torch.bfloat16, L.C64: torch.complex64, L.C128: torch.complex128,
-                   L.I32: torch.int32, L.I64: torch.int64}
+                   L.I32: torch.int32, L.I64: torch.int64, L.BOOL: torch.bool}
     _TORCH2CODE = {v: k for k, v in _CODE2TORCH.items()}
   return _torch
 
@@ -184,18 +185,24 @@ class B200Tensor:
   def __repr__(self):
     return "B200Tensor(shape={}, dtype={}, device={})".format(self.shape, self.dtype, self.t.device)
 
-  # comparisons of 0-d results against python numbers (Lanczos `abs(norm) < delta`)
+  # comparisons: a 0-d tensor against a python number gives a python bool (Lanczos `abs(norm) < delta`); anything with
+  # an axis gives a device bool tensor (InfiniteMPS.canonicalize's `eigvals <= cutoff` mask, infinite_mps.py:239)
+  def _compare(self, o, op, pyop):
+    if self.ndim == 0 and not (getattr(o, "ndim", 0) > 0):
+      return pyop(self.item(), _scalar(o))
+    return _be().compare(op, self, o)
+
   def __lt__(self, o):
-    return self.item() < _scalar(o)
+    return self._compare(o, L.LT, operator.lt)
 
   def __le__(self, o):
-    return self.item() <= _scalar(o)
+    return self._compare(o, L.LE, operator.le)
 
   def __gt__(self, o):
-    return self.item() > _scalar(o)
+    return self._compare(o, L.GT, operator.gt)
 
   def __ge__(self, o):
-    return self.item() >= _scalar(o)
+    return self._compare(o, L.GE, operator.ge)
 
   def __abs__(self):
     return _be().abs(self)
